@@ -12,7 +12,9 @@ The problem has W+1 keyframes: window A = KF 0..W-1 is solved and marginalised o
 timed window consumes), every timed step is window B = KF 1..W.
 metric value = minimizer iterations executed / time, whole job (association and marginalisation amortised into it).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
+--dump-outputs DIR writes what the last timed step returned (see dump_outputs) as DIR/<name>.npy, so that two builds can be
+compared output for output on identical, seeded inputs.
 N>1 is launched by torchrun (one rank per GPU).  The window path does not shard (SURVEY 8e: 20 independent 6x6 blocks and
 a 300x300 solve) -> "replicas only": every rank solves the same window; value is the sum over ranks.  The path that DOES
 shard - the batch scan-to-multiscan solve, by keyframe, one NCCL all-reduce of the pose-block buffers per evaluation - is
@@ -29,6 +31,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark writes nothing into the tree (it may be read-only)
 
 CFG = dict(W=20, Q=100_000, M=1_000_000)
 METRIC = "sliding-window FGO iterations/sec (20 KF, 100k surf pts/scan)"
@@ -65,6 +68,28 @@ def window_factors(spec, first, W):
     prior = spec["prior"] if first == 0 else None
     between = [(i - first, j - first) + tuple(rest) for (i, j, *rest) in spec["between"] if first <= i and j < first + W]
     return prior, between
+
+
+def dump_outputs(out_dir, match_counts, r, prior):
+    """Writes what one window step returns to its caller as float64 arrays, out_dir/<name>.npy: the association's match count
+    per keyframe, the solve's poses, speed-biases, accepted steps, per-iteration log and summary counters (not its timings),
+    and the marginalisation prior handed to the next window.  Under 2 MB at cfg 2: the largest are the prior's two n x n
+    matrices, n <= 15 W."""
+    from glio_b200 import api
+    out = dict(match_counts=match_counts, poses=r["poses"], speed_bias=r["speed_bias"], steps=r["steps"])
+    for name, _ in api.Iteration._fields_:
+        if name != "reserved":
+            out["iteration_" + name] = [it[name] for it in r["iterations"]]
+    s = r["summary"]
+    for name in ("termination", "num_iterations", "num_successful_steps", "num_unsuccessful_steps", "num_evaluations",
+                 "num_jacobian_evaluations", "num_linear_solves", "num_valid_steps", "initial_cost", "final_cost"):
+        out["summary_" + name] = getattr(s, name)
+    pa = prior.arrays()
+    for name in ("lin_jac", "lin_res", "x0_pose", "x0_sb", "A_info", "b_info"):
+        out["prior_" + name] = pa[name]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(v, np.float64))
 
 
 class ClockSampler:
@@ -163,7 +188,6 @@ def run_reference(args, rank, world):
     if rank != 0:
         return
     from oracle import pyoracle as po
-    po.build()
     cores = os.cpu_count() or 1
     P, spec = build_problem()
     q_sub = args.ref_subsample
@@ -447,16 +471,17 @@ def run_glio(args, rank, world, local_rank):
 
     def one_step(m, pending=None):
         ctx.set_map(m)
-        ctx.window_associate(posesB)
+        nm = ctx.window_associate(posesB)
         if pending is not None:
             pending.wait()                           # the previous window's prior is complete before this solve starts
         r = ctx.window_solve(posesB, sb0, hfB, opts, band=band)
         job = ctx.window_marginalize_async(r["poses"], r["speed_bias"], hfB) if pipelined else Done(ctx.window_marginalize(r["poses"], r["speed_bias"], hfB))
-        return len(r["steps"]), r, job
+        return len(r["steps"]), r, job, nm
 
     step_wall = {}
 
     def timed_run(nsteps, sampler=None):
+        """Returns (iterations, device ms, wall s, what the last step returned: match counts, solve result, prior)."""
         iters = 0
         marks = {0, nsteps // 2, nsteps - 1}            # three NVML reads per run: a read stalls the launch queue for 0.5 - 4 ms depending on the box
         ctx.window_set_scans(dscans[1:W + 1])
@@ -471,12 +496,12 @@ def run_glio(args, rank, world, local_rank):
         for si in range(nsteps):
             with torch.cuda.stream(st):
                 flush.fill_(1)                      # L2 flush between steps (256 MB > 126 MB L2), inside the timed region
-            it, _r, job = one_step(dmap, job)
+            it, r, job, nm = one_step(dmap, job)
             iters += it
             if sampler is not None and si in marks:
                 sampler.sample()
             tick.append(time.perf_counter())
-        job.wait()                                  # the last marginalisation completes inside the timed region
+        prior = job.wait()                          # the last marginalisation completes inside the timed region
         e1.record(st)
         torch.cuda.synchronize()
         wall = time.perf_counter() - t0
@@ -488,7 +513,7 @@ def run_glio(args, rank, world, local_rank):
         step_wall.clear()
         step_wall.update(p50=round(float(np.median(per)), 4), mean=round(float(per.mean()), 4), max=round(float(per.max()), 4), argmax=int(per.argmax()), all=[round(float(v), 3) for v in per],
                          mean_of_steps_after_an_nvml_read=round(float(np.mean(after)), 4) if after else None)
-        return iters, ms, wall
+        return iters, ms, wall, (nm, r, prior)
 
     # NVML is initialised and queried during the warm-up steps: the first query of a process can stall the GPU work queue for
     # tens of milliseconds on some boxes (measured: a fixed ~85 ms once per process), which must not land in the timed region.
@@ -504,15 +529,17 @@ def run_glio(args, rank, world, local_rank):
         sampler.reset()
     # (A) the reported value: K steps, inputs resident in HBM, no per-kernel instrumentation
     l0 = ctx.launch_count
-    iters, ms, wall = timed_run(args.steps, sampler)
+    iters, ms, wall, last = timed_run(args.steps, sampler)
     launches = ctx.launch_count - l0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last)
     step_wall_value = dict(step_wall)
     clocks = sampler.result() if sampler else None
     # (B) the same K steps again with every kernel launch bracketed by CUDA events on the launching stream: the
     #     per-kernel durations the roofline uses (its step time is reported next to the value for transparency)
     ctx.lib_profile(True)
     ctx.knn_fallback_queries(reset=True)
-    _, ms_prof, _ = timed_run(args.steps)
+    _, ms_prof, _, _ = timed_run(args.steps)
     prof = ctx.lib_profile_read()
     n_fallback = ctx.knn_fallback_queries()
     ctx.lib_profile(False)
@@ -572,7 +599,7 @@ def run_glio(args, rank, world, local_rank):
         ctx.window_marginalize(rs["poses"], rs["speed_bias"], hfB); t4 = time.perf_counter()
         split = dict(l2_flush_ms=round(1e3 * (t0 - tf), 3), set_map_ms=round(1e3 * (t1 - t0), 3), associate_ms=round(1e3 * (t2 - t1), 3),
                      solve_ms=round(1e3 * (t3 - t2), 3), marginalize_ms=round(1e3 * (t4 - t3), 3))
-    _, rlast, jlast = one_step(dmap)
+    _, rlast, jlast, _ = one_step(dmap)
     plast = jlast.wait()
 
     tmax, tmax_e, it_sum, it_sum_e = ms, ms_e, iters, iters_e
@@ -654,7 +681,6 @@ def run_glio(args, rank, world, local_rank):
     cpu = None; parity = None
     if not args.no_cpu_baseline and world == 1:
         from oracle import pyoracle as po
-        po.build()
         q_sub = args.cpu_subsample
         cores = os.cpu_count() or 1
         tree = po.KdTree(P["map_xyz"])
@@ -712,7 +738,12 @@ def main():
     ap.add_argument("--batch-k", type=int, default=400)
     ap.add_argument("--cpu-subsample", type=int, default=1, help="cpu_baseline leg: use every n-th scan point")
     ap.add_argument("--ref-subsample", type=int, default=1, help="--impl reference: use every n-th scan point")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "glio":
+        ap.error("--dump-outputs is only supported with --impl glio")
     rank = int(os.environ.get("RANK", 0)); world = int(os.environ.get("WORLD_SIZE", 1)); local = int(os.environ.get("LOCAL_RANK", 0))
     if args.impl == "reference":
         run_reference(args, rank, world)

@@ -1,65 +1,69 @@
-"""Pins of the oracle's association pieces to third-party code that IS in this image (VERDICT r1 item 1d).
+"""Pins of the oracle's association pieces to third-party code.
 
 The reference searches with pcl::KdTreeFLANN<PointXYZI>::nearestKSearch (GLIO/src/Estimator.cpp:3647, :3746, :3832) =
-FLANN's KDTreeSingleIndex over L2_Simple<float>, and fits the plane with Eigen's colPivHouseholderQr (:3661).  Neither
-PCL nor Eigen is installed here, but OpenCV's bundled FLANN (cv2.flann_Index; the same FLANN code base: KDTREE_SINGLE =
-KDTreeSingleIndex, LINEAR = brute force; its L2<float> functor accumulates a 3-vector as ((dx*dx) + dy*dy) + dz*dz, the
-same order as L2_Simple) and LAPACK's column-pivoted QR (scipy.linalg.qr(pivoting=True) = dgeqp3) are.  These tests tie
-the oracle's kNN (indices AND float distances, bit for bit) and the 5x3 least-squares solve to those libraries."""
+FLANN's KDTreeSingleIndex over L2_Simple<float>, and fits the plane with Eigen's colPivHouseholderQr (:3661).  The kNN
+tests compare with FLANN's answers recorded from OpenCV's bundled FLANN (tests/golden/flann_knn5.npz, made by
+tests/golden/make_flann_golden.py; the same FLANN code base: KDTREE_SINGLE = KDTreeSingleIndex, LINEAR = brute force; its
+L2<float> functor accumulates a 3-vector as ((dx*dx) + dy*dy) + dz*dz, the same order as L2_Simple).  The plane tests
+compare with LAPACK's column-pivoted QR (scipy.linalg.qr(pivoting=True) = dgeqp3).  These tests tie the oracle's kNN
+(indices AND float distances, bit for bit) and the 5x3 least-squares solve to those libraries."""
+import importlib.util
+import os
+
 import numpy as np
 import pytest
 
 from glio_b200 import synth
 
-cv2 = pytest.importorskip("cv2")
-FLANN_INDEX_LINEAR, FLANN_INDEX_KDTREE_SINGLE = 0, 4
+HERE = os.path.dirname(os.path.abspath(__file__))
 
 
-def _flann_knn5(map_xyz, qry, algorithm):
-    prm = dict(algorithm=algorithm, leaf_max_size=15) if algorithm == FLANN_INDEX_KDTREE_SINGLE else dict(algorithm=algorithm)
-    index = cv2.flann_Index(np.ascontiguousarray(map_xyz, np.float32), prm)
-    idx, sqd = index.knnSearch(np.ascontiguousarray(qry, np.float32), 5, params=dict(checks=-1, eps=0.0, sorted=True))
-    return idx.astype(np.int32), sqd.astype(np.float32)
+@pytest.fixture(scope="module")
+def flann():
+    spec = importlib.util.spec_from_file_location("make_flann_golden", os.path.join(HERE, "golden", "make_flann_golden.py"))
+    mk = importlib.util.module_from_spec(spec); spec.loader.exec_module(mk)
+    return mk, np.load(mk.PATH)
 
 
-def test_knn_matches_flann_kdtree_single_and_linear_small(oracle):
+def _assert_is_flanns_answer(flann, name, map_xyz, qry, idx, sqd):
+    """idx / sqd equal FLANN's recorded answer for these queries: the sampled rows entry by entry, every row by digest."""
+    mk, g = flann
+    assert mk.digest(map_xyz, qry) == str(g[name + "_input_sha256"]), f"{name}: not the map / queries FLANN answered"
+    rows = g[name + "_rows"]
+    assert np.array_equal(idx[rows], g[name + "_idx"]), f"{name}: kNN indices differ from FLANN on the sampled rows"
+    assert np.array_equal(sqd[rows], g[name + "_sqd"]), f"{name}: kNN float distances differ from FLANN on the sampled rows"
+    assert mk.digest(idx) == str(g[name + "_idx_sha256"]), f"{name}: kNN indices differ from FLANN"
+    assert mk.digest(sqd) == str(g[name + "_sqd_sha256"]), f"{name}: kNN float distances differ from FLANN"
+
+
+def test_knn_matches_flann_kdtree_single_and_linear_small(oracle, flann):
     """Small, dense cloud with many near neighbours: FLANN KDTREE_SINGLE == FLANN LINEAR == oracle brute == oracle kd-tree."""
-    P = synth.window_problem(W=2, Q=3000, M=40000, seed=31)
-    t2, q2 = synth.lidar_pose_in_world(P["poses_init"][0, :3], P["poses_init"][0, 3:])
-    pm = oracle.transform_points(P["scans"][0], t2, q2)
-    ib, db, tie = oracle.knn5_brute(P["map_xyz"], pm)
+    map_xyz, pm = flann[0].small_problem()
+    ib, db, tie = oracle.knn5_brute(map_xyz, pm)
     assert not tie.any(), "the generator is supposed to be tie free"
-    ik, dk = oracle.KdTree(P["map_xyz"]).knn5(pm)
-    for algo in (FLANN_INDEX_KDTREE_SINGLE, FLANN_INDEX_LINEAR):
-        fi, fd = _flann_knn5(P["map_xyz"], pm, algo)
-        assert np.array_equal(fi, ib) and np.array_equal(fd, db), f"oracle brute force differs from FLANN algorithm {algo}"
-        assert np.array_equal(fi, ik) and np.array_equal(fd, dk), f"oracle kd-tree differs from FLANN algorithm {algo}"
+    ik, dk = oracle.KdTree(map_xyz).knn5(pm)
+    for algo in flann[0].ALGORITHMS:
+        _assert_is_flanns_answer(flann, "small_" + algo, map_xyz, pm, ib, db)       # oracle brute force
+        _assert_is_flanns_answer(flann, "small_" + algo, map_xyz, pm, ik, dk)       # oracle kd-tree
 
 
-def test_knn_matches_flann_at_full_map_size(oracle):
+def test_knn_matches_flann_at_full_map_size(oracle, flann):
     """cfg-2 map (M = 1 M) and 40 k transformed queries of two scans: the oracle's kd-tree (what every full-size parity test
     uses as its reference) returns FLANN KDTreeSingleIndex's indices and float distances bit for bit."""
-    P = synth.window_problem(W=20, Q=100_000, M=1_000_000, seed=synth.SEED0 + 2)
-    tree = oracle.KdTree(P["map_xyz"])
-    index = cv2.flann_Index(P["map_xyz"], dict(algorithm=FLANN_INDEX_KDTREE_SINGLE, leaf_max_size=15))
-    for k in (3, 17):
-        t2, q2 = synth.lidar_pose_in_world(P["poses_init"][k, :3], P["poses_init"][k, 3:])
-        pm = oracle.transform_points(P["scans"][k][:20000], t2, q2)
+    map_xyz, qry = flann[0].full_problem()
+    tree = oracle.KdTree(map_xyz)
+    for k, pm in qry.items():
         ik, dk = tree.knn5(pm)
-        fi, fd = index.knnSearch(pm, 5, params=dict(checks=-1, eps=0.0, sorted=True))
-        assert np.array_equal(fi.astype(np.int32), ik), "kNN indices differ from FLANN at M = 1M"
-        assert np.array_equal(fd.astype(np.float32), dk), "kNN float distances differ from FLANN at M = 1M"
+        _assert_is_flanns_answer(flann, f"full_scan{k}", map_xyz, pm, ik, dk)
 
 
-def test_assoc_gate_and_indices_consistent_with_flann(oracle):
+def test_assoc_gate_and_indices_consistent_with_flann(oracle, flann):
     """The association's idx5/sqd5 outputs (what the GPU is compared with) are FLANN's, and the radius gate is applied to
     FLANN's 5th SQUARED distance (quirk Q1, Estimator.cpp:3651)."""
-    P = synth.window_problem(W=3, Q=5000, M=60000, seed=77)
-    t2, q2 = synth.lidar_pose_in_world(P["poses_init"][1, :3], P["poses_init"][1, 3:])
-    o = oracle.assoc_scan_to_map(P["map_xyz"], P["scans"][1], t2, q2)
-    fi, fd = _flann_knn5(P["map_xyz"], o["pm"], FLANN_INDEX_KDTREE_SINGLE)
-    assert np.array_equal(o["idx5"], fi) and np.array_equal(o["sqd5"], fd)
-    assert np.array_equal(o["status"] == oracle.GO_FAIL_RADIUS, ~(fd[:, 4].astype(np.float64) < 1.5))
+    map_xyz, scan, t2, q2 = flann[0].assoc_problem()
+    o = oracle.assoc_scan_to_map(map_xyz, scan, t2, q2)
+    _assert_is_flanns_answer(flann, "assoc", map_xyz, o["pm"], o["idx5"], o["sqd5"])
+    assert np.array_equal(o["status"] == oracle.GO_FAIL_RADIUS, ~(o["sqd5"][:, 4].astype(np.float64) < 1.5))
 
 
 def test_plane_solve_matches_lapack_pivoted_qr(oracle):
